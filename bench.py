@@ -22,6 +22,8 @@ frames are registered untimed.
               scans, 20 forced GN iterations) measured the same way on fewer frames, each with its own cpu_baseline
 
 `--impl reference` times only the CPU oracle (the reference itself cannot be built offline, see DESIGN.md).
+`--dump-outputs DIR` writes what the timed path returned for its last step as DIR/<name>.npy (see dump_outputs); the scans
+are seeded, so two builds (or the two arms) run with the same arguments can be compared output for output.
 N > 1 (torchrun): every rank registers the same scans with the keypoints sharded rank/world; the JTJ/JTr sums are
 exchanged inside the persistent GN kernel over NVLink peer mailboxes ("strong" scaling of one frame's latency). Rank 0
 also registers the first frames unsharded and the line carries the sharded-vs-single pose difference.
@@ -36,6 +38,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the tree it runs from (which may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -212,8 +215,9 @@ def workload_config(workload_text, world, seq, first, count, frame_points, keypo
             "icp_iters_per_step": round(iters, 2), "preroll_frames": preroll}
 
 
-def run_oracle(seq, first_timed, steps):
-    """CPU oracle over the same frames; returns (scans/s over the timed steps, per-step ms, F, K, iterations per step)."""
+def run_oracle(seq, first_timed, steps, dump_dir=None):
+    """CPU oracle over the same frames; returns (scans/s over the timed steps, per-step ms, F, K, iterations per step).
+    dump_dir: the outputs of the last timed step are written there."""
     from oracle_lib import oracle
     orc = oracle()
     od = orc.odometry(make_options(orc))
@@ -229,6 +233,8 @@ def run_oracle(seq, first_timed, steps):
             f_sum += sm.num_corrected_points
             k_sum += sm.num_keypoints
             it_sum += sm.icp_summary.num_iters
+    if dump_dir:
+        dump_outputs(dump_dir, od, sm)
     n = max(len(times), 1)
     return len(times) / (sum(times) / 1e3), times, f_sum / n, k_sum / n, it_sum / n
 
@@ -302,8 +308,57 @@ def pose_vector(sm):
                     list(sm.frame.end_pose.quat))
 
 
-def run_native(eng, D, seq, preroll, W, K, n_roof, with_dropin=True, parity_frames=0):
-    """All GPU passes of one workload over `seq`. Returns the fields of the bench line (rank 0) — timing is max over ranks."""
+# summary.npy, in this order: the RegistrationSummary's counters and decisions (its timings are left out: they differ
+# from run to run), then the map size after the step
+SUMMARY_FIELDS = ("success", "sample_size", "number_of_residuals", "robust_level", "points_added", "number_of_attempts",
+                  "num_corrected_points", "num_all_corrected_points", "num_keypoints", "distance_correction",
+                  "relative_distance", "relative_orientation", "ego_orientation", "icp_success", "icp_num_residuals_used",
+                  "icp_num_iters", "map_size")
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, od, sm):
+    """What a caller of RegisterFrame receives for the frame `sm` summarises (the last one `od` registered), as float64
+    DIR/<name>.npy:
+      frame, initial_frame   (2, 8): begin and end pose, each tx ty tz qx qy qz qw dest_timestamp
+      summary                SUMMARY_FIELDS
+      corrected_points, all_corrected_points, keypoints   (n, 8): the summary's point vectors, one WPoint3D per row:
+                             raw xyz, timestamp, world xyz, index_frame
+    """
+    from ct_icp_b200 import _abi as abi
+
+    def frame_rows(f):
+        return np.array([list(p.tr) + list(p.quat) + [p.dest_timestamp] for p in (f.begin_pose, f.end_pose)])
+
+    def points(which):
+        p = od.points(which)
+        return np.column_stack([p["raw"], p["timestamp"], p["world"], p["index_frame"]]).astype(np.float64)
+
+    def summary_value(name):
+        if name == "map_size":
+            return od.MapSize()
+        if name.startswith("icp_"):
+            return getattr(sm.icp_summary, name[len("icp_"):])
+        return getattr(sm, name)
+
+    out = {
+        "frame": frame_rows(sm.frame), "initial_frame": frame_rows(sm.initial_frame),
+        "summary": np.array([summary_value(f) for f in SUMMARY_FIELDS], dtype=np.float64),
+        "corrected_points": points(abi.POINTS_CORRECTED),
+        "all_corrected_points": points(abi.POINTS_ALL_CORRECTED),
+        "keypoints": points(abi.POINTS_KEYPOINTS),
+    }
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("outputs of %d bytes exceed the dump limit of %d" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def run_native(eng, D, seq, preroll, W, K, n_roof, with_dropin=True, parity_frames=0, dump_dir=None):
+    """All GPU passes of one workload over `seq`. Returns the fields of the bench line (rank 0) — timing is max over ranks.
+    dump_dir: rank 0 writes the outputs of pass A's last timed step there."""
     from ct_icp_b200 import _abi as abi
     torch = D.torch
     world, rank, device = D.world, D.rank, D.device
@@ -351,6 +406,8 @@ def run_native(eng, D, seq, preroll, W, K, n_roof, with_dropin=True, parity_fram
         f_sum += sm.num_corrected_points
         iters_sum += t.icp_iterations
     D.barrier()
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, od, sm)
     total_ms = D.max_over_ranks(float(np.sum(step_ms)))
     out = {"value": K / (total_ms / 1e3), "ms_per_step": total_ms / K, "gpu_launches": launches,
            "frame_points": f_sum / K, "keypoints": kp_sum / K, "iters": iters_sum / K}
@@ -457,8 +514,8 @@ def run_native(eng, D, seq, preroll, W, K, n_roof, with_dropin=True, parity_fram
     return out
 
 
-def cpu_baseline_for(seq, first, steps, cores):
-    v, times, f, k, it = run_oracle(seq, first, steps)
+def cpu_baseline_for(seq, first, steps, cores, dump_dir=None):
+    v, times, f, k, it = run_oracle(seq, first, steps, dump_dir)
     threads = oracle_threads()
     return {"value": v, "unit": UNIT, "cores": threads, "kind": "port", "ms_per_step": float(np.mean(times)),
             "sample": "%d timed frames (after %d untimed) of the same sequence; %s; %d host CPUs on this box"
@@ -477,6 +534,8 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[2] / configs[4] extra workloads")
     ap.add_argument("--workload", default="kitti64_gn", choices=sorted(WORKLOADS),
                     help="kitti64_gn is BASELINE.json's metric configuration (the bench line)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned for its last step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
     global _WORKLOAD, WORKLOAD
     _WORKLOAD = args.workload
@@ -495,7 +554,7 @@ def main():
         if rank != 0:
             return 0
         seq = make_scans(first + K, sensor_name)
-        cb, (f, k, it) = cpu_baseline_for(seq, first, K, cores)
+        cb, (f, k, it) = cpu_baseline_for(seq, first, K, cores, args.dump_outputs)
         line = {
             "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": K,
             "warmup": W, "ms_per_step": cb["ms_per_step"], "higher_is_better": True, "scaling": "strong",
@@ -519,7 +578,8 @@ def main():
     clocks = ClockSampler(D.device)
     D.barrier()
     clocks.start()
-    res = run_native(eng, D, seq, preroll, W, K, n_roof, with_dropin=True, parity_frames=6 if world > 1 else 0)
+    res = run_native(eng, D, seq, preroll, W, K, n_roof, with_dropin=True, parity_frames=6 if world > 1 else 0,
+                     dump_dir=args.dump_outputs)
     clock_info = clocks.stop()     # sampled from the start of the device-timed steps to the end of the e2e steps
 
     cpu_baseline = None
