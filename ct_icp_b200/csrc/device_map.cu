@@ -41,6 +41,8 @@ __global__ void k_clear_level(MapLevel L) {
 
 // Phase 1 of InsertPointCloud: find-or-create the voxel of every point and thread the point onto the voxel's
 // candidate list. One thread per point; the list order is arbitrary (phase 2 re-orders by point index).
+// A voxel that already holds B points accepts nothing (map.h:276-291) and its count only changes in phase 2, so its
+// points are neither threaded nor is the voxel touched: phase 2 only visits voxels that can still change.
 __device__ __forceinline__ void insert_claim_dev(const MapLevel &L, MapCounters *ctr, const double *world, int n,
                                                  int *__restrict__ next, uint32_t *__restrict__ touched) {
     const double inv_res = 1.0 / L.res;
@@ -72,6 +74,10 @@ __device__ __forceinline__ void insert_claim_dev(const MapLevel &L, MapCounters 
         }
         if (slot < 0) {
             atomicExch(&ctr->overflow, 1u);
+            next[i] = kNil;
+            continue;
+        }
+        if (L.slots[slot].count >= (uint32_t) L.B) {
             next[i] = kNil;
             continue;
         }
@@ -153,26 +159,36 @@ __device__ __forceinline__ void insert_commit_dev(const MapLevel &L, MapCounters
                 m = 1;
             }
             __syncwarp();
-            for (int a = 0; a < m && count < L.B; ++a) {
-                const int c = s_sorted[w][a];
-                const double lx = world[3 * c] - ox, ly = world[3 * c + 1] - oy, lz = world[3 * c + 2] - oz;
-                bool too_close = false;
-                for (int j = lane; j < count; j += 32) {
-                    const float4 q = s_pts[w][j];
-                    const double dx = (double) q.x - lx, dy = (double) q.y - ly, dz = (double) q.z - lz;
-                    const double d2 = dx * dx + dy * dy + dz * dz;
-                    too_close |= !(d2 > L.min_dist2);
+            for (int a0 = 0; a0 < m && count < L.B; a0 += 32) {
+                // the local coordinates of the next 32 candidates, loaded by the lanes side by side: the sequential rule
+                // below then waits on no global load
+                double cx = 0.0, cy = 0.0, cz = 0.0;
+                if (a0 + lane < m) {
+                    const int c = s_sorted[w][a0 + lane];
+                    cx = world[3 * c] - ox; cy = world[3 * c + 1] - oy; cz = world[3 * c + 2] - oz;
                 }
-                const bool reject = __any_sync(0xffffffffu, too_close);
-                if (!reject) {
-                    if (lane == 0) {
-                        const float4 v = make_float4((float) lx, (float) ly, (float) lz, (float) (frame_ordinal + 1));
-                        s_pts[w][count] = v;
-                        gpts[count] = v;
+                const int chunk = min(32, m - a0);
+                for (int a = 0; a < chunk && count < L.B; ++a) {
+                    const double lx = __shfl_sync(0xffffffffu, cx, a), ly = __shfl_sync(0xffffffffu, cy, a),
+                                 lz = __shfl_sync(0xffffffffu, cz, a);
+                    bool too_close = false;
+                    for (int j = lane; j < count; j += 32) {
+                        const float4 q = s_pts[w][j];
+                        const double dx = (double) q.x - lx, dy = (double) q.y - ly, dz = (double) q.z - lz;
+                        const double d2 = dx * dx + dy * dy + dz * dz;
+                        too_close |= !(d2 > L.min_dist2);
                     }
-                    ++count;
+                    const bool reject = __any_sync(0xffffffffu, too_close);
+                    if (!reject) {
+                        if (lane == 0) {
+                            const float4 v = make_float4((float) lx, (float) ly, (float) lz, (float) (frame_ordinal + 1));
+                            s_pts[w][count] = v;
+                            gpts[count] = v;
+                        }
+                        ++count;
+                    }
+                    __syncwarp();
                 }
-                __syncwarp();
             }
             processed += m;
         }
@@ -280,7 +296,7 @@ struct FusedUpdateArgs {
     const FrameVerdict *verdict;
     double *frame_origins_mut;
 };
-__global__ void __launch_bounds__(kInsertWarps * 32)
+__global__ void __launch_bounds__(kInsertWarps * 32, 4)   // 4 co-resident CTAs per SM (UpdateFused's grid)
 k_map_update_fused(FusedUpdateArgs a) {
     namespace cg = cooperative_groups;
     cg::grid_group grid = cg::this_grid();

@@ -337,7 +337,7 @@ void Engine::IngestImpl(const ScanView &scan, const FrameInfo &info, int64_t sta
     if (n > pipe_->MaxPoints()) throw CapacityError("scan has more points than max_points_per_frame");
 
     // host buffers were packed and their H2D copy enqueued by PackAndUpload (RegisterCommon) before the pose pair existed
-    if (staged_slot >= 0) pipe_->UploadFromDevice(staged_[staged_slot].d_points, staged_[staged_slot].d_lo, n);   // already packed, already in HBM
+    if (staged_slot >= 0) pipe_->UploadFromDevice(staged_[staged_slot].d_points, staged_[staged_slot].d_lo, n);   // read in place
     timing_.h2d_bytes += pipe_->h2d_bytes();
     const double sample_size = k < options_.init_num_frames ? options_.init_voxel_size : options_.voxel_size;
     // frames 0 and 1: every timestamp := end_timestamp (odometry.cpp:355-359)
@@ -767,6 +767,7 @@ int64_t Engine::StageFrame(const ScanView &scan) {
 }
 void Engine::ClearStaged() {
     CT_CUDA_CHECK(cudaSetDevice(device_));
+    pipe_->DetachRaw();   // the last frame's points stay readable (GetPoints) after its staged scan is freed
     CT_CUDA_CHECK(cudaStreamSynchronize(stream_));
     for (auto &sc : staged_) { cudaFree(sc.d_points); cudaFree(sc.d_lo); }
     staged_.clear();

@@ -41,23 +41,44 @@ __device__ __forceinline__ unsigned long long short_voxel_key(const RawPoint &p,
            (unsigned long long) (unsigned short) z;
 }
 
-// claim: every point bids (priority, index) for its voxel
+// find-or-insert `key` in the scratch hash grid (linear probing); returns its slot
+__device__ __forceinline__ uint32_t grid_find_or_insert(unsigned long long *keys, uint32_t cap_mask, unsigned long long key) {
+    uint32_t h = hash_key(key) & cap_mask;
+    while (true) {
+        unsigned long long k = *reinterpret_cast<volatile unsigned long long *>(&keys[h]);
+        if (k == kGridEmpty) k = atomicCAS(&keys[h], kGridEmpty, key);
+        if (k == kGridEmpty || k == key) return h;
+        h = (h + 1) & cap_mask;
+    }
+}
+// claim: every point bids (priority, index) for its voxel. Consecutive scan points share few voxels (a median of 3 keys
+// per warp on a 64-beam scan, up to ~1000 points in one voxel next to the sensor), so the lanes of a warp that hold the
+// same key first agree on their smallest priority and only that lane (the group's leader) probes and bids: one atomic per
+// (warp, voxel) instead of one per point, and no queue of atomics at a hot voxel's word. Priorities are unique, so the
+// bid is the same one the point-by-point claim would have won with. slot_of[i] = the slot for a leader, -1 otherwise
+// (a non-leader can never be its voxel's winner).
+// All lanes of a warp run the same number of iterations (the loop walks whole warps), as the warp collectives require.
 __device__ __forceinline__ void grid_claim_dev(const float4 *pts, const float4 *lo, int n, double voxel_size, int use_perm,
                                                uint64_t seed, uint64_t counter, unsigned long long *keys,
                                                unsigned long long *vals, uint32_t cap_mask, int *__restrict__ slot_of) {
     const Perm perm = perm_make(seed, counter, (uint32_t) max(n, 1));
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const int lane = threadIdx.x & 31;
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, num_warps = (gridDim.x * blockDim.x) >> 5;
+    for (int base = warp * 32; base < n; base += num_warps * 32) {
+        const int i = base + lane;
+        const unsigned active = __ballot_sync(0xffffffffu, i < n);
+        if (i >= n) continue;
         const unsigned long long key = short_voxel_key(load_raw(pts, lo, i), voxel_size);
         const uint32_t prio = use_perm ? perm_apply(perm, (uint32_t) i) : (uint32_t) i;
-        uint32_t h = hash_key(key) & cap_mask;
-        while (true) {
-            unsigned long long k = *reinterpret_cast<volatile unsigned long long *>(&keys[h]);
-            if (k == kGridEmpty) k = atomicCAS(&keys[h], kGridEmpty, key);
-            if (k == kGridEmpty || k == key) break;
-            h = (h + 1) & cap_mask;
+        const unsigned peers = __match_any_sync(active, key);
+        const uint32_t best = __reduce_min_sync(peers, prio);
+        const bool leader = prio == best;
+        uint32_t h = 0;
+        if (leader) {
+            h = grid_find_or_insert(keys, cap_mask, key);
+            atomicMin(&vals[h], ((unsigned long long) prio << 32) | (unsigned) i);
         }
-        atomicMin(&vals[h], ((unsigned long long) prio << 32) | (unsigned) i);
-        slot_of[i] = (int) h;
+        slot_of[i] = leader ? (int) h : -1;
     }
 }
 __global__ void k_grid_claim(const float4 *__restrict__ pts, const float4 *__restrict__ lo, const int *__restrict__ d_n,
@@ -65,15 +86,17 @@ __global__ void k_grid_claim(const float4 *__restrict__ pts, const float4 *__res
                              unsigned long long *vals, uint32_t cap_mask, int *__restrict__ slot_of) {
     grid_claim_dev(pts, lo, *d_n, voxel_size, use_perm, seed, counter, keys, vals, cap_mask, slot_of);
 }
-// mark: winners raise a flag at their position in the permuted order
+// mark: winners raise a flag at their position in the permuted order (slot_of < 0: a point that did not bid)
 __device__ __forceinline__ void grid_mark_dev(int n, int use_perm, uint64_t seed, uint64_t counter,
                                               const unsigned long long *vals, const int *slot_of, uint32_t *__restrict__ flags,
                                               uint32_t *__restrict__ src, uint32_t *__restrict__ tile_count) {
     const Perm perm = perm_make(seed, counter, (uint32_t) max(n, 1));
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const int slot = slot_of[i];
+        if (slot < 0) continue;   // not its warp group's bidder
         const uint32_t prio = use_perm ? perm_apply(perm, (uint32_t) i) : (uint32_t) i;
         const unsigned long long mine = ((unsigned long long) prio << 32) | (unsigned) i;
-        if (vals[slot_of[i]] == mine) {
+        if (vals[slot] == mine) {
             flags[prio] = 1u;
             src[prio] = (uint32_t) i;
             atomicAdd(&tile_count[prio >> kTileShift], 1u);   // integer atomics: order-independent result
@@ -95,13 +118,29 @@ struct EmitScratch {
     uint32_t warp[kTileThreads / 32];
     uint32_t before, total;
 };
+// capacity of the hash grid of a selection over n points (load <= 0.5)
+__device__ __forceinline__ uint32_t grid_cap_for(uint32_t n) {
+    uint32_t cap = 1024;
+    while (cap < 2 * n) cap <<= 1;
+    return cap;
+}
+// The claim of a second, unpermuted selection over the emitted points (grid_sampling of the sub-sampled frame), issued
+// while they are emitted: its priority is the output position, which the emit already holds together with the point.
+// `grid` (keys | vals of grid_cap_for(total) words each) must be clean; `tile` (tile counters | flags of the second
+// selection) is cleared here for total positions.
+struct NextClaim {
+    double voxel_size;
+    unsigned long long *grid;
+    int *slot_of;      // indexed by output position
+    uint32_t *tile;
+};
 // all threads of a CTA of kTileThreads threads; returns the number of winners (identical in every CTA)
 __device__ __forceinline__ uint32_t grid_emit_dev(const float4 *pts, const float4 *lo, const uint32_t *in_src_index, int n,
                                                   const uint32_t *flags, const uint32_t *src, const uint32_t *tile_count,
                                                   int use_perm2, uint64_t seed, uint64_t counter2, int override_alpha,
                                                   float alpha_value, float4 *__restrict__ out, float4 *__restrict__ out_lo,
                                                   uint32_t *__restrict__ out_src_index, int *__restrict__ d_total,
-                                                  EmitScratch &sc) {
+                                                  EmitScratch &sc, const NextClaim *next = nullptr) {
     uint32_t (&s_red)[2][kTileThreads / 32] = sc.red;
     uint32_t (&s_warp)[kTileThreads / 32] = sc.warp;
     uint32_t &s_before = sc.before, &s_total = sc.total;
@@ -123,6 +162,12 @@ __device__ __forceinline__ uint32_t grid_emit_dev(const float4 *pts, const float
     const uint32_t total = s_total;
     if (blockIdx.x == 0 && tid == 0) *d_total = (int) total;
     const Perm perm2 = perm_make(seed, counter2, max(total, 1u));
+    uint32_t next_mask = 0;
+    if (next) {
+        next_mask = grid_cap_for(total) - 1;
+        const size_t words = kMaxTiles + (size_t) total;
+        for (size_t t = (size_t) blockIdx.x * blockDim.x + tid; t < words; t += (size_t) gridDim.x * blockDim.x) next->tile[t] = 0u;
+    }
 
     for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
         uint32_t before = 0;
@@ -166,12 +211,20 @@ __device__ __forceinline__ uint32_t grid_emit_dev(const float4 *pts, const float
                 float4 val = pts[i];
                 if (override_alpha) val.w = alpha_value;
                 out[dst] = val;
+                // (the point as load_raw(out, out_lo, dst) reads it back)
+                RawPoint r{f32_to_f64(val.x), f32_to_f64(val.y), f32_to_f64(val.z), 0.0};
                 if (out_lo) {
                     float4 l = lo ? lo[i] : make_float4(0.f, 0.f, 0.f, 0.f);
                     if (override_alpha) l.w = 0.f;
                     out_lo[dst] = l;
+                    r.x += (double) l.x; r.y += (double) l.y; r.z += (double) l.z;
                 }
                 out_src_index[dst] = in_src_index ? in_src_index[i] : i;
+                if (next) {
+                    const uint32_t h = grid_find_or_insert(next->grid, next_mask, short_voxel_key(r, next->voxel_size));
+                    atomicMin(&next->grid[next_mask + 1 + h], ((unsigned long long) dst << 32) | dst);
+                    next->slot_of[dst] = (int) h;
+                }
             }
             excl += v[k];
         }
@@ -189,19 +242,22 @@ k_grid_emit(const float4 *__restrict__ pts, const float4 *__restrict__ lo, const
                   out, out_lo, out_src_index, d_total, sc);
 }
 
-// ---- both grid selections of a frame (sub_sample_frame N -> F, grid_sampling F -> K) in ONE cooperative launch: seven
-// phases separated by grid barriers instead of six kernels + four memsets. (Each of those kernels lasts 4-11 us for work
-// worth about one: launch ramp, tail, and the dependency on its predecessor; 46 us of a 310 us step in round 1.)
+// ---- both grid selections of a frame (sub_sample_frame N -> F, grid_sampling F -> K) in ONE cooperative launch: five
+// phases separated by four grid barriers (claim 1 | mark 1 | emit 1 + claim 2 | mark 2 | emit 2) instead of six kernels +
+// four memsets. (Each of those kernels lasts 4-11 us for work worth about one: launch ramp, tail, and the dependency on its
+// predecessor; 46 us of a 310 us step in round 1. Each grid barrier costs about 2 us.)
 struct FusedSampleArgs {
     const float4 *raw;
     const float4 *raw_lo;              // residual plane of the scan (nullptr: float32-representable)
     float4 *frame_lo, *kp_lo;          // residual planes of the two selections (written iff raw_lo)
-    int *counts;                       // [0] = N in, [1] = F out, [2] = K out
+    int n;                             // N (also written to counts[0] for later kernels)
+    int *counts;                       // [0] = N, [1] = F out, [2] = K out
     double voxel1, voxel2;
     uint64_t seed, c1, c2;
     int override_alpha;
     float alpha_value;
     unsigned long long *grid;          // keys | vals, 2 * cap1 words
+    unsigned long long *grid2;         // selection 2's keys | vals: claimed into while selection 1 emits, so always clean
     uint32_t cap1;
     int *slot_of;
     uint32_t *tile1, *flags1, *src1;   // selection 1 (tile counters and flags adjacent)
@@ -220,10 +276,12 @@ k_sample_fused(FusedSampleArgs a) {
     cg::grid_group grid = cg::this_grid();
     __shared__ EmitScratch sc;
     const size_t gtid = (size_t) blockIdx.x * blockDim.x + threadIdx.x, gsize = (size_t) gridDim.x * blockDim.x;
-    const int n = a.counts[0];
+    const int n = a.n;
+    if (blockIdx.x == 0 && threadIdx.x == 0) a.counts[0] = n;
     // phase 0: clear the hash grid and the flag / tile-counter arrays of selection 1 (unless the previous launch left them clean)
     if (!a.pre_cleared) {
         for (size_t i = gtid; i < 2 * (size_t) a.cap1; i += gsize) a.grid[i] = kGridEmpty;
+        for (size_t i = gtid; i < 2 * (size_t) a.cap1; i += gsize) a.grid2[i] = kGridEmpty;   // (F <= N: cap2 <= cap1)
         for (size_t i = gtid; i < kMaxTiles + (size_t) n; i += gsize) a.tile1[i] = 0u;   // flags1 = tile1 + kMaxTiles
         grid.sync();
     }
@@ -232,24 +290,22 @@ k_sample_fused(FusedSampleArgs a) {
     grid_mark_dev(n, 1, a.seed, a.c1, a.grid + a.cap1, a.slot_of, a.flags1, a.src1, a.tile1);
     grid.sync();
     float4 *frame_lo = a.raw_lo ? a.frame_lo : nullptr, *kp_lo = a.raw_lo ? a.kp_lo : nullptr;
+    // emit of selection 1 + claim of selection 2 (priority = frame index, grid2) + clear of selection 2's flags; slot_of is
+    // free again (last read by mark 1, a barrier ago)
+    const NextClaim claim2{a.voxel2, a.grid2, a.slot_of, a.tile2};
     const uint32_t F = grid_emit_dev(a.raw, a.raw_lo, nullptr, n, a.flags1, a.src1, a.tile1, 1, a.seed, a.c2, a.override_alpha,
-                                     a.alpha_value, a.frame, frame_lo, a.frame_src, a.counts + 1, sc);
-    // selection 2 works on F points: a smaller grid (the first one is not read any more), its own flags
-    uint32_t cap2 = 1024;
-    while (cap2 < 2 * F) cap2 <<= 1;
-    for (size_t i = gtid; i < 2 * (size_t) cap2; i += gsize) a.grid[i] = kGridEmpty;
-    for (size_t i = gtid; i < kMaxTiles + (size_t) F; i += gsize) a.tile2[i] = 0u;
+                                     a.alpha_value, a.frame, frame_lo, a.frame_src, a.counts + 1, sc, &claim2);
+    const uint32_t cap2 = grid_cap_for(F);
     grid.sync();
-    grid_claim_dev(a.frame, frame_lo, (int) F, a.voxel2, 0, 0, 0, a.grid, a.grid + cap2, cap2 - 1, a.slot_of);
-    grid.sync();
-    grid_mark_dev((int) F, 0, 0, 0, a.grid + cap2, a.slot_of, a.flags2, a.src2, a.tile2);
+    grid_mark_dev((int) F, 0, 0, 0, a.grid2 + cap2, a.slot_of, a.flags2, a.src2, a.tile2);
     grid.sync();
     grid_emit_dev(a.frame, frame_lo, a.frame_src, (int) F, a.flags2, a.src2, a.tile2, 0, 0, 0, 0, 0.f, a.keypoints, kp_lo,
                   a.kp_src, a.counts + 2, sc);
-    // the grid (last read by the mark phase, a barrier ago) and selection 1's arrays (last read by its emit): clean for the
-    // next frame
+    // grid 1 (last read by mark 1), grid 2 (last read by mark 2) and selection 1's arrays (last read by its emit): clean for
+    // the next frame
     if (a.clear_words) {
         for (size_t i = gtid; i < 2 * (size_t) a.cap1; i += gsize) a.grid[i] = kGridEmpty;
+        for (size_t i = gtid; i < 2 * (size_t) cap2; i += gsize) a.grid2[i] = kGridEmpty;
         for (size_t i = gtid; i < (size_t) a.clear_words; i += gsize) a.tile1[i] = 0u;
     }
 }
@@ -385,6 +441,7 @@ FramePipeline::FramePipeline(size_t max_points, cudaStream_t stream) : stream_(s
     CT_CUDA_CHECK(cudaMallocHost(&h_stage_, sizeof(float4) * n));
     CT_CUDA_CHECK(cudaMallocHost(&h_counts_, sizeof(int) * 8));
     CT_CUDA_CHECK(cudaMalloc(&d_raw_, sizeof(float4) * n));
+    raw_ = d_raw_;
     CT_CUDA_CHECK(cudaMalloc(&d_frame_, sizeof(float4) * n));
     CT_CUDA_CHECK(cudaMalloc(&d_keypoints_, sizeof(float4) * n));
     CT_CUDA_CHECK(cudaMalloc(&d_tmp_points_, sizeof(float4) * n));
@@ -410,7 +467,7 @@ FramePipeline::~FramePipeline() {
     cudaFree(d_frame_src_); cudaFree(d_kp_src_); cudaFree(d_tmp_src_);
     cudaFree(d_grid_); cudaFree(d_slot_of_); cudaFree(d_tile_count_); cudaFree(d_src_);
     cudaFree(d_counts_); cudaFree(d_frame_world_); cudaFree(d_all_world_); cudaFree(d_adaptive_);
-    cudaFree(d_tile2_); cudaFree(d_src2_);
+    cudaFree(d_tile2_); cudaFree(d_src2_); cudaFree(d_grid2_);
 }
 
 int FramePipeline::Blocks(size_t n) const { return (int) std::max<size_t>(1, std::min<size_t>((n + 255) / 256, 148 * 8)); }
@@ -428,12 +485,14 @@ void FramePipeline::UploadLo(size_t n) {
     EnsureLo();
     CT_CUDA_CHECK(cudaMemcpyAsync(d_raw_lo_, h_stage_lo_, sizeof(float4) * n, cudaMemcpyHostToDevice, stream_));
     raw_lo_ = true;
+    raw_lo_view_ = d_raw_lo_;
     h2d_bytes_ += sizeof(float4) * n;
 }
 
 void FramePipeline::Upload(size_t n) {
     if (n > max_points_) throw CapacityError("scan has more points than max_points_per_frame");
-    raw_lo_ = frame_lo_ = distorted_ = false;
+    raw_lo_ = frame_lo_ = distorted_ = count_n_pending_ = false;
+    raw_ = d_raw_;
     n_ = n;
     h_counts_[0] = (int) n;
     CT_CUDA_CHECK(cudaMemcpyAsync(d_raw_, h_stage_, sizeof(float4) * n, cudaMemcpyHostToDevice, stream_));
@@ -443,7 +502,8 @@ void FramePipeline::Upload(size_t n) {
 
 void FramePipeline::UploadBegin(size_t n) {
     if (n > max_points_) throw CapacityError("scan has more points than max_points_per_frame");
-    raw_lo_ = frame_lo_ = distorted_ = false;
+    raw_lo_ = frame_lo_ = distorted_ = count_n_pending_ = false;
+    raw_ = d_raw_;
     n_ = n;
     h_counts_[0] = (int) n;
     CT_CUDA_CHECK(cudaMemcpyAsync(d_counts_, h_counts_, sizeof(int), cudaMemcpyHostToDevice, stream_));
@@ -456,17 +516,32 @@ void FramePipeline::UploadRange(size_t begin, size_t end) {
 
 void FramePipeline::UploadFromDevice(const float4 *d_src, const float4 *d_src_lo, size_t n) {
     if (n > max_points_) throw CapacityError("scan has more points than max_points_per_frame");
-    raw_lo_ = frame_lo_ = distorted_ = false;
+    frame_lo_ = distorted_ = false;
     n_ = n;
-    h_counts_[0] = (int) n;
-    CT_CUDA_CHECK(cudaMemcpyAsync(d_raw_, d_src, sizeof(float4) * n, cudaMemcpyDeviceToDevice, stream_));
-    if (d_src_lo) {
+    raw_ = d_src;
+    raw_lo_view_ = d_src_lo;
+    raw_lo_ = d_src_lo != nullptr;
+    count_n_pending_ = true;
+    h2d_bytes_ = 0;
+}
+
+void FramePipeline::DetachRaw() {
+    if (raw_ == d_raw_) return;
+    CT_CUDA_CHECK(cudaMemcpyAsync(d_raw_, raw_, sizeof(float4) * n_, cudaMemcpyDeviceToDevice, stream_));
+    if (raw_lo_) {
         EnsureLo();
-        CT_CUDA_CHECK(cudaMemcpyAsync(d_raw_lo_, d_src_lo, sizeof(float4) * n, cudaMemcpyDeviceToDevice, stream_));
-        raw_lo_ = true;
+        CT_CUDA_CHECK(cudaMemcpyAsync(d_raw_lo_, raw_lo_view_, sizeof(float4) * n_, cudaMemcpyDeviceToDevice, stream_));
     }
+    raw_ = d_raw_;
+    raw_lo_view_ = d_raw_lo_;
+}
+
+void FramePipeline::EnsureCountN() {
+    if (!count_n_pending_) return;
+    h_counts_[0] = (int) n_;
     CT_CUDA_CHECK(cudaMemcpyAsync(d_counts_, h_counts_, sizeof(int), cudaMemcpyHostToDevice, stream_));
-    h2d_bytes_ = sizeof(int);
+    h2d_bytes_ += sizeof(int);
+    count_n_pending_ = false;
 }
 
 void FramePipeline::GridSelect(const float4 *in, const float4 *in_lo, const uint32_t *in_src, const int *d_n_in,
@@ -542,6 +617,8 @@ void FramePipeline::SampleFused(double voxel_size, double sample_voxel_size, uin
     if (!d_tile2_) {
         CT_CUDA_CHECK(cudaMalloc(&d_tile2_, sizeof(uint32_t) * (kMaxTiles + max_points_)));
         CT_CUDA_CHECK(cudaMalloc(&d_src2_, sizeof(uint32_t) * max_points_));
+        CT_CUDA_CHECK(cudaMalloc(&d_grid2_, sizeof(unsigned long long) * 2 * (size_t) grid_cap_));
+        CT_CUDA_CHECK(cudaMemsetAsync(d_grid2_, 0xFF, sizeof(unsigned long long) * 2 * (size_t) grid_cap_, stream_));
         int per_sm = 0;
         CT_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sample_fused, kTileThreads, 0));
         int dev = 0, sms = 148;
@@ -552,8 +629,10 @@ void FramePipeline::SampleFused(double voxel_size, double sample_voxel_size, uin
         fused_grid_ = std::max(1, std::min(per_sm, want) * sms);
     }
     FusedSampleArgs a;
-    a.raw = d_raw_;
+    a.raw = raw_;
     a.raw_lo = d_raw_lo();
+    a.n = (int) n_;
+    count_n_pending_ = false;   // (the launch writes counts[0])
     a.frame_lo = d_frame_lo_; a.kp_lo = d_kp_lo_;
     frame_lo_ = raw_lo_;
     a.counts = d_counts_;
@@ -563,6 +642,7 @@ void FramePipeline::SampleFused(double voxel_size, double sample_voxel_size, uin
     a.override_alpha = override_alpha ? 1 : 0;
     a.alpha_value = alpha_value;
     a.grid = d_grid_;
+    a.grid2 = d_grid2_;
     a.cap1 = std::max<uint32_t>(NextPow2(2 * n_), 1024);
     a.pre_cleared = (preclear_ && clean_cap_ >= a.cap1 && clean_words_ >= kMaxTiles + n_) ? 1 : 0;
     a.clear_words = preclear_ ? (uint32_t) (kMaxTiles + std::min(max_points_, n_ + n_ / 8 + 1024)) : 0u;
@@ -580,7 +660,8 @@ void FramePipeline::SampleFused(double voxel_size, double sample_voxel_size, uin
 
 void FramePipeline::SubSampleFrame(double voxel_size, uint64_t seed, uint64_t counter1, uint64_t counter2,
                                    bool override_alpha, float alpha_value) {
-    GridSelect(d_raw_, d_raw_lo(), nullptr, d_counts_ + 0, n_, voxel_size, 1, seed, counter1, 1, counter2,
+    EnsureCountN();
+    GridSelect(raw_, d_raw_lo(), nullptr, d_counts_ + 0, n_, voxel_size, 1, seed, counter1, 1, counter2,
                override_alpha ? 1 : 0, alpha_value, d_frame_, d_frame_lo_, d_frame_src_, d_counts_ + 1);
     frame_lo_ = raw_lo_;
 }
@@ -636,7 +717,7 @@ void FramePipeline::EnsureAllWorld() {
 }
 void FramePipeline::TransformAll(const Q4 &qb, const V3 &tb, const Q4 &qe, const V3 &te, cudaStream_t stream) {
     EnsureAllWorld();
-    k_transform_points<<<Blocks(n_), 256, 0, stream ? stream : stream_>>>(d_raw_, d_raw_lo(), d_counts_ + 0, qb, tb, qe, te, slerp_consts(qb, qe), d_all_world_);
+    k_transform_points<<<Blocks(n_), 256, 0, stream ? stream : stream_>>>(raw_, d_raw_lo(), d_counts_ + 0, qb, tb, qe, te, slerp_consts(qb, qe), d_all_world_);
     launches_ += 1;
     CT_CUDA_CHECK(cudaGetLastError());
 }

@@ -29,7 +29,7 @@ public:
     bool raw_has_lo() const { return raw_lo_; }
     bool frame_has_lo() const { return frame_lo_; }
     bool frame_distorted() const { return distorted_; }
-    const float4 *d_raw_lo() const { return raw_lo_ ? d_raw_lo_ : nullptr; }
+    const float4 *d_raw_lo() const { return raw_lo_ ? raw_lo_view_ : nullptr; }
     const float4 *d_frame_lo() const { return frame_lo_ ? d_frame_lo_ : nullptr; }
     const float4 *d_keypoints_lo() const { return frame_lo_ ? d_kp_lo_ : nullptr; }
     size_t MaxPoints() const { return max_points_; }
@@ -38,7 +38,11 @@ public:
     // UploadBegin(n), then UploadRange over a partition of [0, n) in any order
     void UploadBegin(size_t n);
     void UploadRange(size_t begin, size_t end);
-    void UploadFromDevice(const float4 *d_src, const float4 *d_src_lo, size_t n);   // scan already packed and resident in HBM
+    // a scan already packed and resident in HBM: the pipeline reads it where it is (no copy) until the next Upload* or
+    // DetachRaw; N reaches the device with the sampler's launch
+    void UploadFromDevice(const float4 *d_src, const float4 *d_src_lo, size_t n);
+    // copy a resident scan the pipeline reads in place into its own buffers (before that scan's memory is freed)
+    void DetachRaw();
 
     // Odometry::InitializeFrame: shuffle → sub_sample_frame → (frames 0,1: timestamp := end) → shuffle
     void SubSampleFrame(double voxel_size, uint64_t seed, uint64_t counter1, uint64_t counter2, bool override_alpha,
@@ -70,7 +74,7 @@ public:
     }
     const int *d_counts() const { return d_counts_; }
 
-    const float4 *d_raw() const { return d_raw_; }
+    const float4 *d_raw() const { return raw_; }
     const float4 *d_frame() const { return d_frame_; }
     const float4 *d_keypoints() const { return d_keypoints_; }
     float4 *d_keypoints_mut() { return d_keypoints_; }
@@ -90,13 +94,13 @@ public:
                     double voxel_size, int use_perm1, uint64_t seed, uint64_t c1, int use_perm2, uint64_t c2,
                     int override_alpha, float alpha_value, float4 *out, float4 *out_lo, uint32_t *out_src, int *d_n_out);
     float4 *d_frame_lo_mut() { EnsureLo(); return d_frame_lo_; }
-    float4 *d_raw_mut() { return d_raw_; }
     double *d_frame_world_mut() { return d_frame_world_; }
     float4 *d_frame_mut() { return d_frame_; }
     uint32_t *d_frame_src_mut() { return d_frame_src_; }
 
 private:
     int Blocks(size_t n) const;
+    void EnsureCountN();   // counts[0] = N on the device, unless the sampler already wrote it
 
     cudaStream_t stream_;
     size_t max_points_, n_ = 0, h2d_bytes_ = 0;
@@ -106,8 +110,10 @@ private:
     float4 *d_raw_ = nullptr, *d_frame_ = nullptr, *d_keypoints_ = nullptr, *d_tmp_points_ = nullptr;
     float4 *h_stage_lo_ = nullptr, *d_raw_lo_ = nullptr, *d_frame_lo_ = nullptr, *d_kp_lo_ = nullptr, *d_tmp_lo_ = nullptr;
     bool raw_lo_ = false, frame_lo_ = false, distorted_ = false;
+    const float4 *raw_ = nullptr, *raw_lo_view_ = nullptr;   // the scan's planes: d_raw_ / d_raw_lo_ or a resident scan
+    bool count_n_pending_ = false;
     uint32_t *d_frame_src_ = nullptr, *d_kp_src_ = nullptr, *d_tmp_src_ = nullptr;
-    unsigned long long *d_grid_ = nullptr;
+    unsigned long long *d_grid_ = nullptr, *d_grid2_ = nullptr;
     int *d_slot_of_ = nullptr;
     uint32_t *d_tile_count_ = nullptr, *d_flags_ = nullptr, *d_src_ = nullptr;   // flags live right after the tile counters
     int *d_counts_ = nullptr;
