@@ -24,6 +24,14 @@ def _as_f64_rows(a, cols):
     return a
 
 
+def _save_blob(b, name, h):
+    size = b.check(b.fn(name)(h, None, 0))
+    buf = C.create_string_buffer(size)
+    written = b.check(b.fn(name)(h, buf, size))
+    assert written == size, (written, size)
+    return buf.raw
+
+
 class Binding:
     def __init__(self, lib, prefix):
         self.lib = lib
@@ -98,6 +106,11 @@ class Binding:
             "odometry_reset_options": (C.c_int, [vp, P(abi.OdometryOptions)]),
             "odometry_enable_sharding": (C.c_int, [vp, vp, C.c_int, C.c_int]),
             "odometry_sharding_mode": (C.c_int, [vp]),
+            "odometry_save_state": (i64, [vp, vp, sz]),
+            "odometry_load_state": (C.c_int, [vp, C.c_char_p, sz]),
+            "odometry_state_options": (C.c_int, [C.c_char_p, sz, P(abi.OdometryOptions)]),
+            "map_save": (i64, [vp, vp, sz]),
+            "map_load": (C.c_int, [vp, C.c_char_p, sz]),
             # oracle only (KAT taps)
             "odometry_last_counters": (None, [vp, P(u64), P(u64)]),
             "neighborhood_describe": (C.c_int, [vp, sz, vp, P(dbl), P(dbl), P(dbl), vp]),
@@ -181,6 +194,13 @@ class Binding:
                                                            out.ctypes.data, len(out)))
         return out[:n].copy()
 
+    def state_options(self, blob):
+        """The effective options stored in an odometry state blob (Odometry.save_state); no device needed."""
+        blob = bytes(blob)
+        o = abi.OdometryOptions()
+        self.check(self.fn("odometry_state_options")(blob, len(blob), C.byref(o)))
+        return o
+
     def permutation(self, seed, counter, n):
         out = np.empty(n, dtype=np.uint32)
         self.check(self.fn("permutation")(seed, counter, n, out.ctypes.data))
@@ -261,6 +281,15 @@ class VoxelMap:
 
     def clear(self):
         self.b.check(self.b.fn("map_clear")(self.h))
+
+    def save(self):
+        """The whole map as a canonical blob (bytes); see include/cticp.h, checkpoint / resume."""
+        return _save_blob(self.b, "map_save", self.h)
+
+    def load(self, blob):
+        """Replaces the map by a blob of `save` (same resolutions and normals; any capacity)."""
+        blob = bytes(blob)
+        self.b.check(self.b.fn("map_load")(self.h, blob, len(blob)))
 
     # CT_ICP_Registration::Register(map, keypoints, frame, motion_model), ct_icp.cpp:1026-1037
     def icp_register(self, icp_options, keypoints, frame, previous_frame=None, motion_options=None,
@@ -465,6 +494,15 @@ class Odometry:
 
     def Reset(self):
         self.b.check(self.b.fn("odometry_reset")(self.h))
+
+    def save_state(self):
+        """Everything that influences the frames to come, as a canonical blob (bytes)."""
+        return _save_blob(self.b, "odometry_save_state", self.h)
+
+    def load_state(self, blob):
+        """Replaces this handle's state by a blob of save_state (options must match, see Binding.state_options)."""
+        blob = bytes(blob)
+        self.b.check(self.b.fn("odometry_load_state")(self.h, blob, len(blob)))
 
     def last_timing(self):
         t = abi.DeviceTiming()

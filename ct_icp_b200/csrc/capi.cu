@@ -7,6 +7,7 @@
 
 #include "../../include/cticp.h"
 #include "engine.h"
+#include "state_io.h"
 
 using namespace cticp;
 
@@ -499,6 +500,31 @@ int cticp_odometry_enable_sharding(cticp_odometry *h, const void *unique_id_128_
 }
 int cticp_odometry_sharding_mode(cticp_odometry *h) { return h->engine->ShardingMode(); }
 
+/* ---- checkpoint / resume (state_io.h) ------------------------------------------------------------------------- */
+int64_t cticp_odometry_save_state(cticp_odometry *h, void *dst, size_t cap) {
+    int64_t size = 0;
+    int rc = Guard([&] {
+        if (!h) throw std::invalid_argument("null handle");
+        size = h->engine->SaveState(static_cast<uint8_t *>(dst), cap);
+        return (int) CTICP_OK;
+    });
+    return rc < 0 ? rc : size;
+}
+int cticp_odometry_load_state(cticp_odometry *h, const void *src, size_t size) {
+    return Guard([&] {
+        if (!h) throw std::invalid_argument("null handle");
+        h->engine->LoadState(static_cast<const uint8_t *>(src), size);
+        return (int) CTICP_OK;
+    });
+}
+int cticp_odometry_state_options(const void *src, size_t size, cticp_odometry_options *out) {
+    return Guard([&] {
+        if (!out) throw std::invalid_argument("null argument");
+        *out = OdoParse(static_cast<const uint8_t *>(src), size, false).options;
+        return (int) CTICP_OK;
+    });
+}
+
 /* ---- Map ----------------------------------------------------------------------------------------------------- */
 int cticp_map_create(const cticp_map_options *options, int device, cticp_map **out) {
     return Guard([&] {
@@ -622,6 +648,26 @@ int cticp_map_radius_search(cticp_map *m, const double *queries_xyz, const doubl
         CAPI_CUDA(cudaMemcpyAsync(out_counts, d_cnt, sizeof(int) * n, cudaMemcpyDeviceToHost, m->stream));
         CAPI_CUDA(cudaStreamSynchronize(m->stream));
         cudaFree(d_q); cudaFree(d_r); cudaFree(d_out); cudaFree(d_cnt);
+        return (int) CTICP_OK;
+    });
+}
+int64_t cticp_map_save(cticp_map *m, void *dst, size_t cap) {
+    int64_t size = 0;
+    int rc = Guard([&] {
+        if (!m) throw std::invalid_argument("null handle");
+        CAPI_CUDA(cudaSetDevice(m->device));
+        size = (int64_t) m->map->Save(static_cast<uint8_t *>(dst), cap);
+        return (int) CTICP_OK;
+    });
+    return rc < 0 ? rc : size;
+}
+int cticp_map_load(cticp_map *m, const void *src, size_t size) {
+    return Guard([&] {
+        if (!m) throw std::invalid_argument("null handle");
+        // the odometry's own map changes together with the trajectory and the policy state that refer to it
+        if (!m->owned) throw UnsupportedError("map load: this map belongs to an odometry; load the odometry's state instead");
+        CAPI_CUDA(cudaSetDevice(m->device));
+        m->map->Load(static_cast<const uint8_t *>(src), size);
         return (int) CTICP_OK;
     });
 }

@@ -7,13 +7,15 @@
 #include "device_map.h"
 
 #include <cooperative_groups.h>
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 #include "gather.cuh"
 #include "frame_policy.h"
+#include "state_io.h"
 
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
-#include <numeric>
 #include <stdexcept>
 #include <vector>
 
@@ -337,49 +339,100 @@ k_map_update_fused(FusedUpdateArgs a) {
     }
 }
 
+// Find-or-create `key` in a table being filled from scratch (keys unique) and copy its run of `count` points and, when
+// both sides keep them, its normal. Shared by the rebuild and by the load of a saved map.
+__device__ __forceinline__ void place_voxel_dev(const MapLevel &dst, unsigned long long key, uint32_t count,
+                                                const float4 *pts, const double *nrm) {
+    uint32_t h = hash_key(key) & dst.cap_mask;
+    for (uint32_t probe = 0; probe <= dst.cap_mask; ++probe) {
+        if (atomicCAS(&dst.slots[h].key, kEmptyKey, key) == kEmptyKey) break;
+        h = (h + 1) & dst.cap_mask;
+    }
+    dst.slots[h].count = count;
+    for (uint32_t j = 0; j < count; ++j) dst.points[(size_t) h * dst.B + j] = pts[j];
+    if (nrm && dst.normals)
+        for (int c = 0; c < 4; ++c) dst.normals[4 * (size_t) h + c] = nrm[c];
+}
+
 // Re-hash the live voxels of `src` into the empty table `dst` (purges tombstones, optionally grows).
 __global__ void k_rebuild(MapLevel src, MapLevel dst, MapCounters *ctr) {
     const uint32_t cap = src.cap_mask + 1;
     for (uint32_t s = blockIdx.x * blockDim.x + threadIdx.x; s < cap; s += gridDim.x * blockDim.x) {
         const unsigned long long key = src.slots[s].key;
         if (key == kEmptyKey || key == kTombKey) continue;
-        uint32_t h = hash_key(key) & dst.cap_mask;
-        for (uint32_t probe = 0; probe <= dst.cap_mask; ++probe) {
-            if (atomicCAS(&dst.slots[h].key, kEmptyKey, key) == kEmptyKey) break;
-            h = (h + 1) & dst.cap_mask;
-        }
-        const uint32_t count = src.slots[s].count;
-        dst.slots[h].count = count;
-        for (uint32_t j = 0; j < count; ++j) dst.points[(size_t) h * dst.B + j] = src.points[(size_t) s * src.B + j];
-        if (src.normals && dst.normals)
-            for (int c = 0; c < 4; ++c) dst.normals[4 * (size_t) h + c] = src.normals[4 * (size_t) s + c];
+        place_voxel_dev(dst, key, src.slots[s].count, src.points + (size_t) s * src.B,
+                        src.normals ? src.normals + 4 * (size_t) s : nullptr);
     }
     (void) ctr;
 }
 
-// Export: every stored point as fp64 world xyz + voxel coords + index within its voxel.
-__global__ void k_export(MapLevel L, unsigned long long *cursor, double *xyz, int *voxel, int *idx_in_voxel,
-                         unsigned long long cap_points) {
+// ---- canonical order of a level (export, save): the live voxels compacted, sorted by packed key on the device, their
+// point runs at the exclusive scan of the counts. Ascending packed key is lexicographic (x, y, z): the bias makes every
+// 21-bit field non-negative. The compaction's order depends on atomic timing; the sort removes it.
+// (`room` entries of output, the live-voxel counter: the host checks the final cursor against it)
+__global__ void k_live_slots(MapLevel L, unsigned long long *keys, uint32_t *slots, unsigned room, unsigned int *cursor) {
     const uint32_t cap = L.cap_mask + 1;
     for (uint32_t s = blockIdx.x * blockDim.x + threadIdx.x; s < cap; s += gridDim.x * blockDim.x) {
         const unsigned long long key = L.slots[s].key;
         if (key == kEmptyKey || key == kTombKey) continue;
-        const uint32_t count = L.slots[s].count;
-        if (!count) continue;
+        const unsigned i = atomicAdd(cursor, 1u);
+        if (i >= room) continue;
+        keys[i] = key;
+        slots[i] = s;
+    }
+}
+__global__ void k_sorted_counts(MapLevel L, const uint32_t *__restrict__ slots, size_t V, uint32_t *counts,
+                                unsigned long long *counts64) {
+    for (size_t i = blockIdx.x * (size_t) blockDim.x + threadIdx.x; i < V; i += (size_t) gridDim.x * blockDim.x) {
+        const uint32_t c = L.slots[slots[i]].count;
+        counts[i] = c;
+        counts64[i] = c;
+    }
+}
+// one warp per voxel run: the dense point runs (and normals) of a save, in key order
+__global__ void k_gather_runs(MapLevel L, const uint32_t *__restrict__ slots, const uint32_t *__restrict__ counts,
+                              const unsigned long long *__restrict__ offsets, size_t V, float4 *out_pts, double *out_normals) {
+    const int lane = threadIdx.x & 31;
+    const size_t warps = (size_t) gridDim.x * (blockDim.x >> 5);
+    for (size_t v = (blockIdx.x * (size_t) blockDim.x + threadIdx.x) >> 5; v < V; v += warps) {
+        const size_t s = slots[v];
+        const uint32_t c = counts[v];
+        const unsigned long long o = offsets[v];
+        for (uint32_t j = lane; j < c; j += 32) out_pts[o + j] = L.points[s * L.B + j];
+        if (out_normals && lane < 4) out_normals[4 * v + lane] = L.normals[4 * s + lane];
+    }
+}
+// one warp per voxel run: GetMapPoints as fp64 world xyz + voxel coordinates, in key order
+__global__ void k_export_runs(MapLevel L, const unsigned long long *__restrict__ keys, const uint32_t *__restrict__ slots,
+                              const uint32_t *__restrict__ counts, const unsigned long long *__restrict__ offsets, size_t V,
+                              double *xyz, int *voxel) {
+    const int lane = threadIdx.x & 31;
+    const size_t warps = (size_t) gridDim.x * (blockDim.x >> 5);
+    for (size_t v = (blockIdx.x * (size_t) blockDim.x + threadIdx.x) >> 5; v < V; v += warps) {
         int vx, vy, vz;
-        unpack_voxel(key, vx, vy, vz);
-        unsigned long long base = atomicAdd(cursor, (unsigned long long) count);
-        for (uint32_t j = 0; j < count; ++j) {
-            unsigned long long o = base + j;
-            if (o >= cap_points) break;
-            const float4 p = L.points[(size_t) s * L.B + j];
+        unpack_voxel(keys[v], vx, vy, vz);
+        const size_t s = slots[v];
+        const uint32_t c = counts[v];
+        const unsigned long long o0 = offsets[v];
+        for (uint32_t j = lane; j < c; j += 32) {
+            const unsigned long long o = o0 + j;
+            const float4 p = L.points[s * L.B + j];
             xyz[3 * o] = vx * L.res + (double) p.x;
             xyz[3 * o + 1] = vy * L.res + (double) p.y;
             xyz[3 * o + 2] = vz * L.res + (double) p.z;
             voxel[3 * o] = vx; voxel[3 * o + 1] = vy; voxel[3 * o + 2] = vz;
-            idx_in_voxel[o] = (int) j;
         }
     }
+}
+__global__ void k_widen_counts(const uint32_t *__restrict__ counts, size_t V, unsigned long long *counts64) {
+    for (size_t i = blockIdx.x * (size_t) blockDim.x + threadIdx.x; i < V; i += (size_t) gridDim.x * blockDim.x) counts64[i] = counts[i];
+}
+// load of a saved level into an empty table: one thread per voxel, like the rebuild
+__global__ void k_place_runs(MapLevel dst, const unsigned long long *__restrict__ keys, const uint32_t *__restrict__ counts,
+                             const unsigned long long *__restrict__ offsets, size_t V, const float4 *__restrict__ pts,
+                             const double *__restrict__ normals) {
+    for (size_t v = blockIdx.x * (size_t) blockDim.x + threadIdx.x; v < V; v += (size_t) gridDim.x * blockDim.x)
+        place_voxel_dev(dst, keys[v], counts[v], pts + offsets[v], normals ? normals + 4 * v : nullptr);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -398,15 +451,19 @@ DeviceMap::DeviceMap(const cticp_map_options &options, cudaStream_t stream, bool
         const auto &rp = options.resolutions[i];
         if (!(rp.resolution > 0) || rp.max_num_points < 1 || rp.max_num_points > kMaxB)
             throw std::invalid_argument("map resolution / max_num_points out of the supported range (1..64)");
-        // default capacity: enough for a 100 m local map at load <= 0.5; tables double on demand (MaintainTables)
-        uint64_t cap = options.capacity_voxels ? options.capacity_voxels : (rp.resolution < 0.5 ? (1ull << 20) : (1ull << 18));
-        AllocLevel(levels_[i], NextPow2(std::max<uint64_t>(cap, 1024)), rp);
+        AllocLevel(levels_[i], (uint32_t) InitialCapacity(rp), rp);
     }
     CT_CUDA_CHECK(cudaMalloc(&d_counters_, sizeof(MapCounters) * levels_.size()));
     CT_CUDA_CHECK(cudaMemsetAsync(d_counters_, 0, sizeof(MapCounters) * levels_.size(), stream_));
     CT_CUDA_CHECK(cudaMalloc(&d_scalar_, 64));
     CT_CUDA_CHECK(cudaMallocHost(&h_counters_, sizeof(MapCounters) * CTICP_MAX_RESOLUTIONS));
     memset(h_counters_, 0, sizeof(MapCounters) * CTICP_MAX_RESOLUTIONS);
+}
+
+// default capacity: enough for a 100 m local map at load <= 0.5; tables double on demand (MaintainTables)
+uint64_t DeviceMap::InitialCapacity(const cticp_resolution_param &rp) const {
+    const uint64_t cap = options_.capacity_voxels ? options_.capacity_voxels : (rp.resolution < 0.5 ? (1ull << 20) : (1ull << 18));
+    return NextPow2(std::max<uint64_t>(cap, 1024));
 }
 
 DeviceMap::~DeviceMap() {
@@ -689,44 +746,214 @@ void DeviceMap::SearchParams(double radius, int *level, int *voxel_neighborhood)
     *voxel_neighborhood = (int) std::ceil(radius / options_.resolutions[idx].resolution);
 }
 
+// ---- canonical order, save, load ---------------------------------------------------------------------------------
+template <typename T>
+struct DeviceBuffer {   // scratch of one call, stream-ordered: no device-wide synchronisation on allocation or release
+    T *p = nullptr;
+    cudaStream_t stream;
+    DeviceBuffer(size_t n, cudaStream_t s) : stream(s) {
+        CT_CUDA_CHECK(cudaMallocAsync((void **) &p, sizeof(T) * std::max<size_t>(n, 1), stream));
+    }
+    ~DeviceBuffer() { cudaFreeAsync(p, stream); }
+    DeviceBuffer(const DeviceBuffer &) = delete;
+    DeviceBuffer &operator=(const DeviceBuffer &) = delete;
+};
+
+static int GridFor(size_t n, int threads) { return (int) std::max<size_t>(1, std::min<size_t>((n + threads - 1) / threads, 148 * 8)); }
+
+// offsets[i] = counts[0] + ... + counts[i - 1] (counts64: the counts widened to 64 bit); returns the total (synchronises)
+static uint64_t ExclusiveScan(const unsigned long long *counts64, const uint32_t *counts, unsigned long long *offsets, size_t V,
+                              cudaStream_t stream) {
+    if (V == 0) return 0;
+    size_t tmp_bytes = 0;
+    CT_CUDA_CHECK(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts64, offsets, (int) V, stream));
+    DeviceBuffer<uint8_t> tmp(tmp_bytes, stream);
+    CT_CUDA_CHECK(cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, counts64, offsets, (int) V, stream));
+    unsigned long long last_off = 0;
+    uint32_t last_count = 0;
+    CT_CUDA_CHECK(cudaMemcpyAsync(&last_off, offsets + V - 1, sizeof(last_off), cudaMemcpyDeviceToHost, stream));
+    CT_CUDA_CHECK(cudaMemcpyAsync(&last_count, counts + V - 1, sizeof(last_count), cudaMemcpyDeviceToHost, stream));
+    CT_CUDA_CHECK(cudaStreamSynchronize(stream));
+    return last_off + last_count;
+}
+
+struct DeviceMap::SortedLevel {   // the live voxels of one level in ascending key order
+    SortedLevel(size_t n, cudaStream_t s) : keys(n, s), slots(n, s), counts(n, s), counts64(n, s), offsets(n, s) {}
+    DeviceBuffer<unsigned long long> keys;
+    DeviceBuffer<uint32_t> slots, counts;
+    DeviceBuffer<unsigned long long> counts64, offsets;
+    size_t V = 0;
+    uint64_t P = 0;
+};
+
+std::unique_ptr<DeviceMap::SortedLevel> DeviceMap::SortLevel(int level, size_t num_voxels) {
+    const MapLevel &L = levels_[level];
+    const size_t cap = (size_t) L.cap_mask + 1;
+    auto S = std::make_unique<SortedLevel>(num_voxels, stream_);
+    DeviceBuffer<unsigned long long> keys_in(num_voxels, stream_);
+    DeviceBuffer<uint32_t> slots_in(num_voxels, stream_);
+    DeviceBuffer<unsigned int> cursor(1, stream_);
+    CT_CUDA_CHECK(cudaMemsetAsync(cursor.p, 0, sizeof(unsigned int), stream_));
+    k_live_slots<<<GridFor(cap, 256), 256, 0, stream_>>>(L, keys_in.p, slots_in.p, (unsigned) num_voxels, cursor.p);
+    CT_CUDA_CHECK(cudaGetLastError());
+    unsigned int V = 0;
+    CT_CUDA_CHECK(cudaMemcpyAsync(&V, cursor.p, sizeof(V), cudaMemcpyDeviceToHost, stream_));
+    CT_CUDA_CHECK(cudaStreamSynchronize(stream_));
+    if (V != num_voxels)
+        throw std::runtime_error("map level " + std::to_string(level) + ": " + std::to_string(V) + " live voxels, the counter says " +
+                                 std::to_string(num_voxels));
+    S->V = V;
+    if (V == 0) return S;
+    size_t tmp_bytes = 0;
+    // bit 63 of a packed key is always 0
+    CT_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, keys_in.p, S->keys.p, slots_in.p, S->slots.p, (int) V, 0, 63,
+                                                  stream_));
+    DeviceBuffer<uint8_t> tmp(tmp_bytes, stream_);
+    CT_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(tmp.p, tmp_bytes, keys_in.p, S->keys.p, slots_in.p, S->slots.p, (int) V, 0, 63,
+                                                  stream_));
+    k_sorted_counts<<<GridFor(V, 256), 256, 0, stream_>>>(L, S->slots.p, V, S->counts.p, S->counts64.p);
+    CT_CUDA_CHECK(cudaGetLastError());
+    S->P = ExclusiveScan(S->counts64.p, S->counts.p, S->offsets.p, V, stream_);
+    return S;
+}
+
 size_t DeviceMap::Export(int level, std::vector<double> &xyz, std::vector<int> &voxels) {
     const MapCounters *c = SyncCounters();
     const size_t n = (size_t) c[level].num_points;
     xyz.assign(3 * n, 0.0);
     voxels.assign(3 * n, 0);
     if (n == 0) return 0;
-    double *d_xyz;
-    int *d_vox, *d_idx;
-    unsigned long long *d_cursor;
-    CT_CUDA_CHECK(cudaMalloc(&d_xyz, sizeof(double) * 3 * n));
-    CT_CUDA_CHECK(cudaMalloc(&d_vox, sizeof(int) * 3 * n));
-    CT_CUDA_CHECK(cudaMalloc(&d_idx, sizeof(int) * n));
-    CT_CUDA_CHECK(cudaMalloc(&d_cursor, sizeof(unsigned long long)));
-    CT_CUDA_CHECK(cudaMemsetAsync(d_cursor, 0, sizeof(unsigned long long), stream_));
-    k_export<<<592, 256, 0, stream_>>>(levels_[level], d_cursor, d_xyz, d_vox, d_idx, n);
-    std::vector<double> hx(3 * n);
-    std::vector<int> hv(3 * n), hi(n);
-    CT_CUDA_CHECK(cudaMemcpyAsync(hx.data(), d_xyz, sizeof(double) * 3 * n, cudaMemcpyDeviceToHost, stream_));
-    CT_CUDA_CHECK(cudaMemcpyAsync(hv.data(), d_vox, sizeof(int) * 3 * n, cudaMemcpyDeviceToHost, stream_));
-    CT_CUDA_CHECK(cudaMemcpyAsync(hi.data(), d_idx, sizeof(int) * n, cudaMemcpyDeviceToHost, stream_));
+    auto S = SortLevel(level, c[level].num_voxels);
+    if (S->P != n) throw std::runtime_error("map level " + std::to_string(level) + ": the voxel runs hold " + std::to_string(S->P) +
+                                            " points, the counter " + std::to_string(n));
+    DeviceBuffer<double> d_xyz(3 * n, stream_);
+    DeviceBuffer<int> d_vox(3 * n, stream_);
+    k_export_runs<<<GridFor(32 * S->V, 256), 256, 0, stream_>>>(levels_[level], S->keys.p, S->slots.p, S->counts.p, S->offsets.p,
+                                                                 S->V, d_xyz.p, d_vox.p);
+    CT_CUDA_CHECK(cudaGetLastError());
+    CT_CUDA_CHECK(cudaMemcpyAsync(xyz.data(), d_xyz.p, sizeof(double) * 3 * n, cudaMemcpyDeviceToHost, stream_));
+    CT_CUDA_CHECK(cudaMemcpyAsync(voxels.data(), d_vox.p, sizeof(int) * 3 * n, cudaMemcpyDeviceToHost, stream_));
     CT_CUDA_CHECK(cudaStreamSynchronize(stream_));
-    cudaFree(d_xyz); cudaFree(d_vox); cudaFree(d_idx); cudaFree(d_cursor);
-    // deterministic order: (voxel x, y, z, index in voxel) — same as the oracle's sorted export
-    std::vector<size_t> order(n);
-    std::iota(order.begin(), order.end(), 0);
-    std::sort(order.begin(), order.end(), [&](size_t a, size_t b) {
-        for (int d = 0; d < 3; ++d)
-            if (hv[3 * a + d] != hv[3 * b + d]) return hv[3 * a + d] < hv[3 * b + d];
-        return hi[a] < hi[b];
-    });
-    for (size_t o = 0; o < n; ++o) {
-        size_t s = order[o];
-        for (int d = 0; d < 3; ++d) {
-            xyz[3 * o + d] = hx[3 * s + d];
-            voxels[3 * o + d] = hv[3 * s + d];
-        }
-    }
     return n;
+}
+
+size_t DeviceMap::Save(uint8_t *dst, size_t cap) {
+    CT_CUDA_CHECK(cudaStreamSynchronize(stream_));
+    // the counters are read privately: the host copy MaintainTables works from stays what the last frame left
+    std::vector<MapCounters> c(levels_.size());
+    CT_CUDA_CHECK(cudaMemcpyAsync(c.data(), d_counters_, sizeof(MapCounters) * c.size(), cudaMemcpyDeviceToHost, stream_));
+    CT_CUDA_CHECK(cudaStreamSynchronize(stream_));
+    MapBlobLayout B;
+    B.num_levels = (int) levels_.size();
+    B.has_normals = with_normals_;
+    B.frame_count = frame_count_;
+    for (int l = 0; l < B.num_levels; ++l) {
+        const auto &rp = options_.resolutions[l];
+        B.levels[l].resolution = rp.resolution;
+        B.levels[l].min_distance = rp.min_distance_between_points;
+        B.levels[l].max_num_points = rp.max_num_points;
+        B.levels[l].V = c[l].num_voxels;
+        B.levels[l].P = c[l].num_points;
+    }
+    MapLayoutFill(B);
+    if (!dst || cap < B.total) return B.total;
+    if (with_normals_ && frame_count_)
+        CT_CUDA_CHECK(cudaMemcpyAsync(dst + B.off_origins, d_frame_origins_, sizeof(double) * 3 * frame_count_,
+                                      cudaMemcpyDeviceToHost, stream_));
+    for (int l = 0; l < B.num_levels; ++l) {
+        const MapBlobLevel &v = B.levels[l];
+        auto S = SortLevel(l, v.V);
+        if (S->P != v.P)
+            throw std::runtime_error("map level " + std::to_string(l) + ": the voxel runs hold " + std::to_string(S->P) +
+                                     " points, the counter says " + std::to_string(v.P));
+        if (v.V == 0) continue;
+        DeviceBuffer<float4> pts(v.P, stream_);
+        DeviceBuffer<double> nrm(with_normals_ ? 4 * v.V : 0, stream_);
+        k_gather_runs<<<GridFor(32 * v.V, 256), 256, 0, stream_>>>(levels_[l], S->slots.p, S->counts.p, S->offsets.p, v.V, pts.p,
+                                                                    with_normals_ ? nrm.p : nullptr);
+        CT_CUDA_CHECK(cudaGetLastError());
+        CT_CUDA_CHECK(cudaMemcpyAsync(dst + v.off_keys, S->keys.p, 8 * v.V, cudaMemcpyDeviceToHost, stream_));
+        CT_CUDA_CHECK(cudaMemcpyAsync(dst + v.off_counts, S->counts.p, 4 * v.V, cudaMemcpyDeviceToHost, stream_));
+        if (v.P) CT_CUDA_CHECK(cudaMemcpyAsync(dst + v.off_points, pts.p, 16 * v.P, cudaMemcpyDeviceToHost, stream_));
+        if (with_normals_) CT_CUDA_CHECK(cudaMemcpyAsync(dst + v.off_normals, nrm.p, 32 * v.V, cudaMemcpyDeviceToHost, stream_));
+    }
+    CT_CUDA_CHECK(cudaStreamSynchronize(stream_));
+    MapWriteHeaders(dst, B);
+    SealBlob(dst, B.total);
+    return B.total;
+}
+
+void DeviceMap::Load(const uint8_t *src, size_t size) {
+    const MapBlobLayout B = MapParse(src, size);
+    if (B.num_levels != (int) levels_.size())
+        throw std::invalid_argument("map load: the blob has " + std::to_string(B.num_levels) + " resolutions, this map " +
+                                    std::to_string(levels_.size()));
+    if (B.has_normals != with_normals_)
+        throw std::invalid_argument(std::string("map load: the blob ") + (B.has_normals ? "keeps" : "does not keep") +
+                                    " per-voxel normals, this map " + (with_normals_ ? "does" : "does not"));
+    for (int l = 0; l < B.num_levels; ++l) {
+        const auto &rp = options_.resolutions[l];
+        const MapBlobLevel &v = B.levels[l];
+        const std::string lv = "map load: resolutions[" + std::to_string(l) + "].";
+        if (v.resolution != rp.resolution) throw std::invalid_argument(lv + "resolution differs");
+        if (v.max_num_points != rp.max_num_points) throw std::invalid_argument(lv + "max_num_points differs");
+        if (v.min_distance != rp.min_distance_between_points) throw std::invalid_argument(lv + "min_distance_between_points differs");
+    }
+    CT_CUDA_CHECK(cudaStreamSynchronize(stream_));
+    // fresh tables at load factor <= 0.5 (MaintainTables' rule); the old ones are released only once all are placed
+    std::vector<MapLevel> fresh(levels_.size(), MapLevel{});
+    try {
+        for (int l = 0; l < B.num_levels; ++l) {
+            const MapBlobLevel &v = B.levels[l];
+            uint64_t cap = InitialCapacity(options_.resolutions[l]);
+            while (v.V * 2 > cap) cap *= 2;
+            if (cap > (1ull << 31)) throw CapacityError("map load: more voxels than a table can hold");
+            AllocLevel(fresh[l], (uint32_t) cap, options_.resolutions[l]);
+            if (v.V == 0) continue;
+            DeviceBuffer<unsigned long long> keys(v.V, stream_), counts64(v.V, stream_), offsets(v.V, stream_);
+            DeviceBuffer<uint32_t> counts(v.V, stream_);
+            DeviceBuffer<float4> pts(v.P, stream_);
+            DeviceBuffer<double> nrm(with_normals_ ? 4 * v.V : 0, stream_);
+            CT_CUDA_CHECK(cudaMemcpyAsync(keys.p, src + v.off_keys, 8 * v.V, cudaMemcpyHostToDevice, stream_));
+            CT_CUDA_CHECK(cudaMemcpyAsync(counts.p, src + v.off_counts, 4 * v.V, cudaMemcpyHostToDevice, stream_));
+            if (v.P) CT_CUDA_CHECK(cudaMemcpyAsync(pts.p, src + v.off_points, 16 * v.P, cudaMemcpyHostToDevice, stream_));
+            if (with_normals_) CT_CUDA_CHECK(cudaMemcpyAsync(nrm.p, src + v.off_normals, 32 * v.V, cudaMemcpyHostToDevice, stream_));
+            k_widen_counts<<<GridFor(v.V, 256), 256, 0, stream_>>>(counts.p, v.V, counts64.p);
+            CT_CUDA_CHECK(cudaGetLastError());
+            ExclusiveScan(counts64.p, counts.p, offsets.p, v.V, stream_);
+            k_place_runs<<<GridFor(v.V, 256), 256, 0, stream_>>>(fresh[l], keys.p, counts.p, offsets.p, v.V, pts.p,
+                                                                 with_normals_ ? nrm.p : nullptr);
+            CT_CUDA_CHECK(cudaGetLastError());
+        }
+        if (with_normals_ && B.frame_count > frame_capacity_) {
+            size_t fcap = std::max<size_t>(4096, frame_capacity_);
+            while (fcap < B.frame_count) fcap *= 2;
+            double *origins = nullptr;
+            CT_CUDA_CHECK(cudaMalloc(&origins, sizeof(double) * 3 * fcap));
+            cudaFree(d_frame_origins_);
+            d_frame_origins_ = origins;
+            frame_capacity_ = fcap;
+        }
+    } catch (...) {
+        for (auto &L : fresh) FreeLevel(L);
+        throw;
+    }
+    for (int l = 0; l < B.num_levels; ++l) {
+        FreeLevel(levels_[l]);
+        levels_[l] = fresh[l];
+        MapCounters &c = h_counters_[l];
+        c = MapCounters{};
+        c.num_points = B.levels[l].P;
+        c.num_voxels = (unsigned int) B.levels[l].V;
+    }
+    if (with_normals_ && B.frame_count)
+        CT_CUDA_CHECK(cudaMemcpyAsync(d_frame_origins_, src + B.off_origins, sizeof(double) * 3 * B.frame_count,
+                                      cudaMemcpyHostToDevice, stream_));
+    CT_CUDA_CHECK(cudaMemcpyAsync(d_counters_, h_counters_, sizeof(MapCounters) * levels_.size(), cudaMemcpyHostToDevice, stream_));
+    CT_CUDA_CHECK(cudaStreamSynchronize(stream_));
+    frame_count_ = B.frame_count;
+    dirty_ = false;
+    readback_pending_ = false;
 }
 
 }  // namespace cticp

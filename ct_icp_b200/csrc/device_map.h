@@ -1,6 +1,7 @@
 // device_map.h — host-side owner of the device-resident voxel map (see device_map.cuh for the layout).
 #pragma once
 #include <cstring>
+#include <memory>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -68,11 +69,21 @@ public:
 
     // GetMapPoints (map.h:354-376) in (voxel, insertion) order; returns the point count
     size_t Export(int level, std::vector<double> &xyz, std::vector<int> &voxels);
+    // the map blob of state_io.h (canonical: voxels in ascending key order). Returns its size; writes only when
+    // cap >= size. Synchronises the stream; the map itself is not changed.
+    size_t Save(uint8_t *dst, size_t cap);
+    // replaces the whole map by a validated blob of the same layout (levels, resolutions, normals); a rejected blob
+    // (std::invalid_argument) leaves the map untouched
+    void Load(const uint8_t *src, size_t size);
 
     int launches() const { return launches_; }
     int rebuilds() const { return rebuilds_; }
 
 private:
+    struct SortedLevel;
+    // canonical order of the `num_voxels` live voxels (the level's counter; synchronises)
+    std::unique_ptr<SortedLevel> SortLevel(int level, size_t num_voxels);
+    uint64_t InitialCapacity(const cticp_resolution_param &rp) const;
     void AllocLevel(MapLevel &L, uint32_t cap, const cticp_resolution_param &rp);
     void RebuildLevel(size_t i, uint64_t new_cap);
     void FreeLevel(MapLevel &L);

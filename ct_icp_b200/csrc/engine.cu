@@ -1,5 +1,6 @@
 // engine.cu — host orchestration of the B200-native odometry (see engine.h).
 #include "engine.h"
+#include "state_io.h"
 
 #include <algorithm>
 #include <atomic>
@@ -202,6 +203,85 @@ void Engine::Reset() {   // odometry.cpp:956-965
     egress_valid_[0] = egress_valid_[1] = egress_valid_[2] = false;
     tail_event_valid_ = false;
     staging_in_flight_ = false;
+}
+
+int64_t Engine::SaveState(uint8_t *dst, size_t cap) {
+    CT_CUDA_CHECK(cudaSetDevice(device_));
+    // the speculative map update of the last frame and the egress of its vectors; the flags that order the next frame
+    // behind them stay as they are (they are satisfied now)
+    CT_CUDA_CHECK(cudaStreamSynchronize(stream_));
+    if (egress_stream_) CT_CUDA_CHECK(cudaStreamSynchronize(egress_stream_));
+    const size_t T = trajectory_.size();
+    const size_t map_size = map_->Save(nullptr, 0);
+    const size_t total = OdoBlobSize(T, map_size);
+    if (!dst || cap < total) return (int64_t) total;
+    OdoHostRecord h{};
+    h.registered_frames = registered_frames_;
+    h.last_num_keypoints = (int64_t) last_num_keypoints_;
+    h.next_robust_level = next_robust_level_;
+    h.robust_num_consecutive_failures = robust_num_consecutive_failures_;
+    h.suspect_registration_error = suspect_registration_error_ ? 1 : 0;
+    h.tracker_skipped_frames = tracker_.skipped_frames;
+    h.tracker_total_insertions = tracker_.total_insertions;
+    h.tracker_cum_distance = tracker_.cum_distance;
+    h.tracker_cum_orientation = tracker_.cum_orientation;
+    h.default_motion_model_present = default_motion_model_.present ? 1 : 0;
+    h.default_motion_model_options = default_motion_model_.options;
+    h.default_motion_model_previous_frame = FrameToC(default_motion_model_.previous_frame);
+    h.trajectory_size = T;
+    std::vector<cticp_frame> tr(T);
+    for (size_t i = 0; i < T; ++i) tr[i] = FrameToC(trajectory_[i]);
+    OdoWrite(dst, options_, h, tr.data(), map_size);
+    map_->Save(dst + OdoBlobSize(T, 0), map_size);
+    SealBlob(dst, total);
+    return (int64_t) total;
+}
+
+void Engine::LoadState(const uint8_t *src, size_t size) {
+    CT_CUDA_CHECK(cudaSetDevice(device_));
+    if (shard_world_ > 1) throw UnsupportedError("load_state: restoring a sharded handle is not supported");
+    const OdoBlobView v = OdoParse(src, size, true);
+    const std::string diff = FirstOptionDifference(v.options, options_);
+    if (!diff.empty()) throw std::invalid_argument("load_state: option " + diff + " differs from this handle's");
+    const OdoHostRecord &h = v.host;
+    if (h.next_robust_level < 0 || h.next_robust_level > options_.robust_minimal_level + 2)
+        throw std::invalid_argument("state blob rejected: next_robust_level " + std::to_string(h.next_robust_level));
+    std::vector<HostFrame> trajectory(h.trajectory_size);
+    for (size_t i = 0; i < trajectory.size(); ++i) {
+        cticp_frame f;
+        memcpy(&f, v.trajectory + i, sizeof(f));
+        trajectory[i] = FrameFromC(f);
+    }
+    // as Reset(): nothing in flight may still read or write the state that is replaced
+    CT_CUDA_CHECK(cudaStreamSynchronize(stream_));
+    if (egress_stream_) CT_CUDA_CHECK(cudaStreamSynchronize(egress_stream_));
+    map_->Load(v.map, v.map_size);   // validates the map blob before it touches the map
+    trajectory_ = std::move(trajectory);
+    registered_frames_ = (int) h.registered_frames;
+    last_num_keypoints_ = (size_t) h.last_num_keypoints;
+    next_robust_level_ = h.next_robust_level;
+    robust_num_consecutive_failures_ = h.robust_num_consecutive_failures;
+    suspect_registration_error_ = h.suspect_registration_error != 0;
+    tracker_.skipped_frames = h.tracker_skipped_frames;
+    tracker_.total_insertions = h.tracker_total_insertions;
+    tracker_.cum_distance = h.tracker_cum_distance;
+    tracker_.cum_orientation = h.tracker_cum_orientation;
+    default_motion_model_.present = h.default_motion_model_present != 0;
+    default_motion_model_.options = h.default_motion_model_options;
+    default_motion_model_.previous_frame = FrameFromC(h.default_motion_model_previous_frame);
+    // the point vectors of the last registered frame are not state: get_points answers as on a new handle
+    pipe_->ForgetFrame();
+    last_frame_ = HostFrame();
+    last_info_ = FrameInfo();
+    frame_world_valid_ = last_all_world_valid_ = last_kp_world_valid_ = keypoints_in_summary_ = false;
+    scan_in_staging_ = false;
+    egress_pending_ = false;
+    egress_valid_[0] = egress_valid_[1] = egress_valid_[2] = false;
+    tail_event_valid_ = false;
+    staging_in_flight_ = false;
+    // LastTiming reads these once a frame was registered: recorded, they read as an empty interval
+    for (int i = 0; i < 4; ++i) CT_CUDA_CHECK(cudaEventRecord(ev_[i], stream_));
+    CT_CUDA_CHECK(cudaStreamSynchronize(stream_));
 }
 
 void Engine::SetSummaryPoints(int mask) {

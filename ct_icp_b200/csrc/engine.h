@@ -114,6 +114,11 @@ public:
     const std::vector<HostFrame> &Trajectory() const { return trajectory_; }
     int64_t MapSize();
     void Reset();
+    // checkpoint / resume (state_io.h): everything that influences the frames to come. SaveState returns the blob size
+    // and writes only when cap >= size; it waits for the work in flight and leaves the handle as it was. LoadState
+    // replaces the whole state (also of a handle that registered frames already); a rejected blob changes nothing.
+    int64_t SaveState(uint8_t *dst, size_t cap);
+    void LoadState(const uint8_t *src, size_t size);
     DeviceMap &Map() { return *map_; }
     IcpSolver &Solver() { return *icp_; }
     cudaStream_t Stream() const { return stream_; }

@@ -73,6 +73,11 @@ public:
         for (int i = 0; i < 4; ++i) h_counts_[i] = c[i];
     }
     const int *d_counts() const { return d_counts_; }
+    // no frame registered yet, as on a new pipeline (N and the host counters zero)
+    void ForgetFrame() {
+        n_ = 0;
+        for (int i = 0; i < 4; ++i) h_counts_[i] = 0;
+    }
 
     const float4 *d_raw() const { return raw_; }
     const float4 *d_frame() const { return d_frame_; }

@@ -13,6 +13,7 @@
 // (`pose.quat`, `pose.tr`, `dest_timestamp`, `RawPoint()`, `WorldPoint()`, `Timestamp()`): this header has no
 // dependency besides cticp.h. INTEGRATION.md shows the variant that keeps the reference's own headers.
 #pragma once
+#include <algorithm>
 #include <array>
 #include <cmath>
 #include <cstdint>
@@ -316,6 +317,21 @@ public:
         if (!callbacks_.empty()) cticp_check(cticp_odometry_set_callback(h_, &Odometry::Trampoline, this));
     }
     std::shared_ptr<MapView> GetMapPointer() { return std::make_shared<MapView>(cticp_odometry_map(h_)); }            // :272
+    // checkpoint / resume (new; cticp.h): a handle created with StateOptions(blob) that loads the blob continues the
+    // saved run bit for bit
+    std::vector<uint8_t> SaveState() const {
+        const int64_t n = cticp_odometry_save_state(h_, nullptr, 0);
+        cticp_check((int) std::min<int64_t>(n, 0));
+        std::vector<uint8_t> blob((size_t) n);
+        cticp_check((int) std::min<int64_t>(cticp_odometry_save_state(h_, blob.data(), blob.size()), 0));
+        return blob;
+    }
+    void LoadState(const std::vector<uint8_t> &blob) { cticp_check(cticp_odometry_load_state(h_, blob.data(), blob.size())); }
+    static OdometryOptions StateOptions(const std::vector<uint8_t> &blob) {
+        OdometryOptions o;
+        cticp_check(cticp_odometry_state_options(blob.data(), blob.size(), &o));
+        return o;
+    }
     const OdometryOptions &Options() const { return options_; }
     cticp_odometry *handle() const { return h_; }
 

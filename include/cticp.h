@@ -427,6 +427,33 @@ int cticp_odometry_enable_sharding(cticp_odometry *h, const void *unique_id_128_
 /* 0 = not sharded, 1 = exchange through ncclAllReduce, 2 = in-kernel exchange over peer mailboxes */
 int cticp_odometry_sharding_mode(cticp_odometry *h);
 
+/* ---- checkpoint / resume (new; the reference has no checkpoint of odometry state, SURVEY §5) ---------------
+ * A blob holds everything that influences the frames to come: the effective options (after the motion-compensation
+ * overrides of the constructor), the trajectory, the robust-registration ladder, the insertion tracker, the default
+ * motion model, the keypoint-count hint of the ICP kernels, and the device map (voxel keys, fp32 point runs, per-voxel
+ * normals, begin position of every inserted frame). A run saved after frame k and loaded into a new handle produces the
+ * same bits for every later frame as the run that never stopped. The point vectors of the last registered frame are
+ * not state: after a load the get_points / write_points calls answer as on a new handle.
+ * Layout (little-endian, sections 8-byte aligned; DESIGN.md §9 has every field):
+ *   odometry: "CTICPODO", u32 version, u32 sizeof(cticp_odometry_options), u64 total_bytes, u64 checksum, options,
+ *             host-state record, cticp_frame trajectory[T], one map blob
+ *   map:      "CTICPMAP", u32 version, u32 num_levels, u64 total_bytes, u64 checksum, u32 has_normals, u32 0,
+ *             u64 frame_count, [f64 frame_origins[3 * frame_count]], per level: f64 resolution, f64 min_distance,
+ *             i32 max_num_points, i32 0, u64 V, u64 P, u64 keys[V] (ascending), u32 counts[V] (padded to 8 bytes),
+ *             float4 points[P], [f64 normals[4 * V]]
+ *   checksum: FNV-1a 64 over bytes [32, total_bytes) read as u64 words (guards against truncation and corruption).
+ * Blobs are canonical: voxels in ascending packed-key order, points in insertion order inside a voxel, so saving the
+ * same state twice gives the same bytes.
+ * save: returns the blob size and writes only when cap >= size; waits for the work in flight, changes nothing.
+ * load: replaces the handle's whole state (also after frames were registered). Options must be equal except
+ * map_options.capacity_voxels and max_points_per_frame (CTICP_ERR_INVALID_ARGUMENT names the first differing field);
+ * the tables are sized for the loaded map. Any rejected blob leaves the handle untouched. A sharded handle can save,
+ * but its load fails with CTICP_ERR_UNSUPPORTED. */
+int64_t cticp_odometry_save_state(cticp_odometry *h, void *dst, size_t cap);
+int cticp_odometry_load_state(cticp_odometry *h, const void *src, size_t size);
+/* the options stored in an odometry blob (no device needed): create the handle to load the blob into from them */
+int cticp_odometry_state_options(const void *src, size_t size, cticp_odometry_options *out);
+
 /* device timing of the last register_frame (CUDA events on the handle's stream), milliseconds */
 typedef struct cticp_device_timing {
     double total_ms;
@@ -492,6 +519,11 @@ int cticp_map_radius_search(cticp_map *m, const double *queries_xyz, const doubl
                             int32_t *out_counts);
 /* ClearMap(), include/ct_icp/map.h:296 */
 int cticp_map_clear(cticp_map *m);
+/* the map blob above, alone (new). load requires equal resolutions, max_num_points, min_distance_between_points and
+ * the same choice of keeping per-voxel normals (select_valid_normals_direction); capacity may differ. A map that
+ * belongs to an odometry can be saved but not loaded (CTICP_ERR_UNSUPPORTED): load the odometry's state instead. */
+int64_t cticp_map_save(cticp_map *m, void *dst, size_t cap);
+int cticp_map_load(cticp_map *m, const void *src, size_t size);
 
 /* ---- Registration (L3 boundary) ------------------------------------------------------------------------- */
 
